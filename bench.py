@@ -20,6 +20,9 @@ and reported separately as `optimizer` / `train_step`.
 
 `value` is measured with inputs resident in HBM (CUDA-graph replay); `e2e` runs the same step from pinned HOST buffers
 through the engine API (H2D of the batch and D2H of the loss inside the timed region). Prints ONE JSON line.
+
+`--dump-outputs DIR` writes what the last timed step returned (outputs, loss and parameter gradient of every plan) to DIR as
+.npy files. Inputs and weights are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -130,13 +133,12 @@ class ClockSampler:
 
 
 # ---------------------------------------------------------------------------------------------- CPU arm
-def run_cpu_reference(cfgj, B, Nv, Nt, steps, warmup, budget_s=90.0, threads=None):
+def run_cpu_reference(cfgj, B, Nv, Nt, steps, warmup, budget_s=None, threads=None):
     """The reference algorithm's VILBertForVLTasks fwd + VQA loss + bwd, fp32, on the host cores, at a FIXED sample batch B:
-    `warmup` untimed steps (>= 1, so that allocator / thread-pool start-up never lands in a timed step), then up to `steps` timed
-    steps (>= 3 unless the time budget runs out first). Uses the unmodified reference when $VILBERT_REFERENCE_ROOT (default
-    /root/reference) holds it (kind "reference"), else the oracle port, which is bit-identical to it on CPU (kind "port")."""
+    `warmup` untimed steps (>= 1, so that allocator / thread-pool start-up never lands in a timed step), then `steps` timed
+    steps, fewer only if `budget_s` seconds have passed. Runs the oracle port (kind "port"), which tests/test_oracle_golden.py
+    holds bit-exact to the reference's recorded outputs and gradients on CPU."""
     import torch
-    from oracle import ref_loader
     from oracle import vilbert_oracle as O
     if threads is None:
         try:
@@ -149,48 +151,29 @@ def run_cpu_reference(cfgj, B, Nv, Nt, steps, warmup, budget_s=90.0, threads=Non
     P = O.synth_params(cfg, seed=0)
     inp = O.synth_inputs(cfg, B, Nv, Nt, seed=1234)
     tgt = O.synth_vqa_target(B, 3129)
-    kind = "port"
-    model = None
-    if ref_loader.available() and os.environ.get("VB_CPU_ARM", "") != "port":
-        try:
-            ref = ref_loader.load()
-            model = ref.VILBertForVLTasks(ref.BertConfig.from_dict(cfgj), num_labels=1, default_gpu=False)
-            model.load_state_dict(P, strict=False)
-            model.train()
-            kind = "reference"
-        except Exception as e:   # noqa: BLE001
-            print(f"[bench] reference import failed ({e}); timing the oracle port", file=sys.stderr)
-            model = None
-    if model is None:
-        Pg = {k: v.clone().requires_grad_(True) for k, v in P.items() if k != "cls.predictions.decoder.weight"}
-        Pg["cls.predictions.decoder.weight"] = Pg["bert.embeddings.word_embeddings.weight"]
+    Pg = {k: v.clone().requires_grad_(True) for k, v in P.items() if k != "cls.predictions.decoder.weight"}
+    Pg["cls.predictions.decoder.weight"] = Pg["bert.embeddings.word_embeddings.weight"]
 
     def one_step():
         t0 = time.perf_counter()
-        if model is not None:
-            model.zero_grad()
-            out = model(inp["input_txt"], inp["input_imgs"], inp["image_loc"], inp["token_type_ids"], inp["attention_mask"], inp["image_attention_mask"],
-                        inp["co_attention_mask"], inp["task_ids"])
-            O.vqa_loss(out[0], tgt).backward()
-        else:
-            for v in Pg.values():
-                v.grad = None
-            _, heads = O.vilbert_for_vl_tasks(Pg, cfg, inp["input_txt"], inp["input_imgs"], inp["image_loc"], inp["token_type_ids"], inp["attention_mask"],
-                                              inp["image_attention_mask"], inp["co_attention_mask"], inp["task_ids"])
-            O.vqa_loss(heads[0], tgt).backward()
+        for v in Pg.values():
+            v.grad = None
+        _, heads = O.vilbert_for_vl_tasks(Pg, cfg, inp["input_txt"], inp["input_imgs"], inp["image_loc"], inp["token_type_ids"], inp["attention_mask"],
+                                          inp["image_attention_mask"], inp["co_attention_mask"], inp["task_ids"])
+        O.vqa_loss(heads[0], tgt).backward()
         return time.perf_counter() - t0
 
     t_start = time.perf_counter()
     for _ in range(max(warmup, 1)):
         one_step()
     times = []
-    for _ in range(max(steps, 3)):
+    for _ in range(steps):
         times.append(one_step())
-        if len(times) >= 1 and time.perf_counter() - t_start > budget_s:
+        if budget_s is not None and time.perf_counter() - t_start > budget_s:
             break
     sec = sum(times) / len(times)
-    return dict(value=B * Nv * Nt / sec, unit="pairs/s", cores=threads, kind=kind, sec_per_step=sec, sample_batch=B, steps_timed=len(times),
-                sample=f"{'the unmodified reference' if kind == 'reference' else 'oracle port (bit-exact vs the reference on CPU)'}: VILBertForVLTasks fwd + VQA loss + "
+    return dict(value=B * Nv * Nt / sec, unit="pairs/s", cores=threads, kind="port", sec_per_step=sec, sample_batch=B, steps_timed=len(times),
+                sample=f"oracle port (bit-exact vs the reference on CPU): VILBertForVLTasks fwd + VQA loss + "
                        f"bwd, fp32, fixed B={B} x {Nv} regions x {Nt} tokens, {max(warmup, 1)} warm-up + {len(times)} timed step(s), {threads} threads")
 
 
@@ -222,6 +205,34 @@ def synth_loss_inputs(plan, kind, seed, torch):
         out["image_target"] = torch.softmax(torch.randn(plan.B, plan.Nv - 1, plan.cfg.v_target_size, generator=g), -1)
         out["next_sentence_label"] = torch.randint(0, 2, (plan.B,), generator=g)
     return out
+
+
+DUMP_BYTES = 60 * 2 ** 20    # all arrays of --dump-outputs together, leaving room for the .npy headers below 64 MB
+
+
+def dump_outputs(out_dir, T, eng, torch):
+    """What the timed step hands its caller after the last run, as float32 .npy files: every output of each plan
+    (`<task>.<output>.npy`), its loss (`<task>.loss.npy`) and the flat fp32 parameter gradient (`param_grad.npy`, accumulated over
+    every step of the run). An array larger than its equal share of DUMP_BYTES is replaced by a 1-D sample of it, at sorted
+    flat indices drawn from a CPU generator seeded with 0, so the same arguments select the same elements on every build.
+    With a shared activation arena only the plan that ran last still holds its outputs; the others contribute their loss."""
+    import numpy as np
+    arrays = {}
+    for t in T:
+        plan = t["plan"]
+        if eng.arena is None or eng.arena_owner[0] is plan:
+            for name, x in plan.outputs.items():
+                arrays[f"{t['name']}.{name}"] = x
+        arrays[f"{t['name']}.loss"] = plan.loss
+    arrays["param_grad"] = eng.ps.grad
+    cap = DUMP_BYTES // 4 // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        x = x.detach()
+        if x.numel() > cap:
+            idx = torch.randint(0, x.numel(), (cap,), generator=torch.Generator().manual_seed(0)).sort().values
+            x = x.reshape(-1)[idx.to(x.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), x.float().cpu().numpy())
 
 
 def main():
@@ -256,7 +267,13 @@ def main():
     ap.add_argument("--no-module-api", action="store_true", help="skip the VILBertForVLTasks.forward -> loss.backward() leg")
     ap.add_argument("--cpu-batch", type=int, default=8)
     ap.add_argument("--profile-ops", action="store_true", help="print the per-kernel-class time table to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs, loss and parameter gradient of the last timed step to DIR "
+                                                          "as float32 .npy files (a fixed sample of each large array; rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -277,7 +294,7 @@ def main():
             return
         W = max(min(a.warmup, 2), 1)
         c2 = load_config_json("bert_base_6layer_6conect")
-        r = run_cpu_reference(c2, a.cpu_batch, 100, 36, max(min(a.steps, 5), 3), W, budget_s=120.0)
+        r = run_cpu_reference(c2, a.cpu_batch, 100, 36, a.steps, W)
         print(json.dumps({"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "pairs/s", "n_gpus": a.gpus, "steps": r["steps_timed"], "warmup": W,
                           "ms_per_step": r["sec_per_step"] * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
                           "data": "synthetic", "config": {"workload": "config 2: bert_base_6layer_6conect VQA-shape synthetic, 100 regions x 36 tokens, all heads + VQA BCE loss, fwd+bwd",
@@ -447,6 +464,8 @@ def main():
     ms = timed(lambda i: step(), a.steps)
     clocks.mark_end()
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, T, eng, torch)     # before the legs below change the weights, inputs and gradients
     ms_step = ms / a.steps
     loss_val = float(sum(t["plan"].loss.item() for t in T))
     # ---------------- the same step followed by the fused optimizer (AdamW + 16-bit weight copies + gradient zeroing in one launch)

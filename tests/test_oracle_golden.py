@@ -46,6 +46,11 @@ def test_oracle_matches_reference_tensors(name, golden_dir):
     for k, v in gold["heads"].items():
         assert rel(heads_o[k], v) < 1e-5, k
     for k, v in gold["grads"].items():
+        if k.endswith(("key.bias", "key1.bias", "key2.bias")):
+            # zero in exact arithmetic (the softmax over the keys ignores a shift common to all of them): both tensors hold
+            # rounding noise whose bits depend on the CPU's vector width, so the difference is scaled by the key weight's gradient
+            assert (Pg[k].grad - v).abs().max() <= 1e-5 * gold["grads"][k[:-4] + "weight"].abs().max(), k
+            continue
         assert rel(Pg[k].grad, v) < 1e-5, k
     # q_dense1/2 never receive a gradient (vilbert.py:834,841)
     assert all(Pg[k].grad is None for k in Pg if "q_dense" in k)
